@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the movement-primitive black-box rollout path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch: B = 65,536 episodes per GPU of
 fancy_ProMP/HoleReacher-v0 (BASELINE.json configs[1]) = trajectory generation + velocity controller
@@ -23,6 +23,10 @@ Prints ONE JSON line (see README / DESIGN.md "Measurement" for the keys):
 Multi-GPU (torchrun, one rank per GPU): the env batch is sharded, no data-path collective; per-step returns /
 lengths / flags reach every rank inside the timed region — stored by the rollout kernel itself into peer-mapped gather buffers
 over NVLink (FG_BENCH_EXCHANGE=nccl: an overlapped ncclAllGather instead) ("scaling": "weak").
+
+--dump-outputs DIR writes what the last timed step of `value` returned (rank 0's envs) as DIR/<name>.npy: the arrays step()
+hands its caller (obs, return, terminated, truncated, is_success, is_collided, end_effector, trajectory_length).  The inputs
+are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -43,6 +47,25 @@ SIGMA = 0.25
 CPU_BATCH = 64                   # envs per oracle call in the CPU baseline (numpy-vectorised port)
 OPS_PER_ENV_STEP = 4356          # SURVEY.md §8d, HoleReacher/ProMP (FMA = 2, each collision test once per step)
 TRAJ_BYTES_PER_ENV = 2 * 200 * 5 * 4 + N_PARAMS * 4   # fg_trajgen: pos + vel out, params in
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays, limit_bytes=DUMP_LIMIT_BYTES):
+    """Writes `arrays` (numpy, one row per env) as out_dir/<name>.npy: float32 and boolean arrays as float32, all others as
+    float64 (exact for the int32 lengths).  If they would take more than `limit_bytes`, the same seeded sample of env rows
+    is written from every array, and the chosen rows go to env_index.npy."""
+    import numpy as np
+    out = {k: np.asarray(v, dtype=np.float32 if v.dtype in (np.float32, np.bool_) else np.float64) for k, v in arrays.items()}
+    n = len(next(iter(out.values())))
+    row_bytes = sum(v[0].nbytes for v in out.values())
+    budget = limit_bytes - 128 * (len(out) + 1)          # room for the .npy headers
+    if n * row_bytes > budget:
+        idx = np.sort(np.random.default_rng(0).choice(n, budget // (row_bytes + 8), replace=False))
+        out = {k: v[idx] for k, v in out.items()}
+        out["env_index"] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
 
 
 def ncu_numbers():
@@ -238,7 +261,12 @@ def main():
     ap.add_argument("--envs-per-gpu", type=int, default=B_PER_GPU)
     ap.add_argument("--sigma", type=float, default=SIGMA)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     args.warmup = max(args.warmup, 3)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -417,6 +445,13 @@ def main():
         t_end.record()
         host_issue_ms = (time.perf_counter() - host_t0) * 1e3 / K     # host time to ISSUE one step (no sync inside)
         sync_all()
+    last_outputs = None
+    if args.dump_outputs and rank == 0:
+        # the result buffers of the last timed launch, copied before later launches of the ring overwrite them
+        te, tr, success, collided = env._flag_bytes
+        outs = {"obs": env._obs, "return": env._ret, "terminated": te, "truncated": tr, "is_success": success,
+                "is_collided": collided, "end_effector": env._info[:, 0:2], "trajectory_length": env._len}
+        last_outputs = {k: x.cpu().numpy() for k, x in outs.items()}
     if world > 1:
         clk.__exit__()
     elapsed_ms = t_start.elapsed_time(t_end)
@@ -826,6 +861,8 @@ def main():
                     episodes_per_s=episodes_per_s, mean_episode_length=env_steps / (K * B), host_issue_ms_per_step=host_issue_ms,
                     roofline=roofline, roofline_trajgen=roofline_traj, cpu_baseline=cpu, e2e=e2e, e2e_sync=e2e_sync, e2e_graph=e2e_graph,
                     clocks=clocks, gpu_launches=K, configs=extras)
+        if last_outputs is not None:
+            dump_outputs(args.dump_outputs, last_outputs)
         emit(line)
     if world > 1:
         dist.destroy_process_group()

@@ -1,9 +1,12 @@
-"""bench.py contract checks that need no GPU: the reference arm prints ONE JSON line with the agreed keys; the argument
-parser accepts the driver's flags."""
+"""bench.py contract checks: the reference arm prints ONE JSON line with the agreed keys; the argument parser accepts
+the documented flags; --dump-outputs writes the outputs of the last timed step (end to end on the GPU)."""
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -30,6 +33,51 @@ def test_reference_arm_other_ranks_exit_quietly():
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2", "--steps", "1",
                           "--warmup", "1"], capture_output=True, text=True, timeout=120, cwd=ROOT, env=env)
     assert out.returncode == 0 and out.stdout.strip() == ""
+
+
+def test_steps_below_one_are_refused():
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "0"],
+                         capture_output=True, text=True, timeout=120, cwd=ROOT)
+    assert out.returncode == 2 and "--steps" in out.stderr and out.stdout == ""
+
+
+def test_dump_outputs_writes_floats_and_a_seeded_sample_above_the_limit(tmp_path):
+    import bench
+    rng = np.random.default_rng(1)
+    B = 1000
+    arrays = {"obs": rng.standard_normal((B, 18)).astype(np.float32), "return": rng.standard_normal(B),
+              "terminated": rng.random(B) < 0.5, "trajectory_length": rng.integers(1, 201, B).astype(np.int32)}
+    bench.dump_outputs(str(tmp_path / "all"), arrays)
+    assert sorted(os.listdir(tmp_path / "all")) == sorted(k + ".npy" for k in arrays)
+    for k, v in arrays.items():
+        got = np.load(tmp_path / "all" / f"{k}.npy")
+        assert got.dtype in (np.float32, np.float64) and np.array_equal(got, v), k
+    limit = 40_000
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), arrays, limit_bytes=limit)
+        assert sum(os.path.getsize(tmp_path / d / f) for f in os.listdir(tmp_path / d)) <= limit
+    idx = np.load(tmp_path / "a" / "env_index.npy")
+    assert 0 < len(idx) < B and (np.diff(idx) > 0).all()
+    for k, v in arrays.items():
+        assert np.array_equal(np.load(tmp_path / "a" / f"{k}.npy"), v[idx.astype(np.int64)]), k
+        assert np.array_equal(np.load(tmp_path / "a" / f"{k}.npy"), np.load(tmp_path / "b" / f"{k}.npy")), k
+
+
+@pytest.mark.gpu
+def test_bench_dumps_the_outputs_of_its_last_timed_step(tmp_path):
+    B = 16384
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--gpus", "1", "--steps", "2", "--warmup", "1",
+                          "--envs-per-gpu", str(B), "--no-cpu-baseline", "--dump-outputs", str(tmp_path)],
+                         capture_output=True, text=True, timeout=900, cwd=ROOT)
+    assert out.returncode == 0, out.stderr[-2000:]
+    d = json.loads(out.stdout)
+    assert d["steps"] == 2 and d["gpu_launches"] == 2
+    got = {f[:-len(".npy")]: np.load(tmp_path / f) for f in os.listdir(tmp_path)}
+    assert set(got) == {"obs", "return", "terminated", "truncated", "is_success", "is_collided", "end_effector", "trajectory_length"}
+    assert all(v.dtype in (np.float32, np.float64) and len(v) == B for v in got.values())
+    assert got["obs"].ndim == 2 and got["end_effector"].shape == (B, 2)
+    length = got["trajectory_length"]
+    assert ((length >= 1) & (length <= 200)).all() and np.isfinite(got["return"]).all()
 
 
 def test_ncu_numbers_json_is_what_the_committed_summaries_say():
