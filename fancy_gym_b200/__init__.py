@@ -14,7 +14,7 @@ from .envs.registry import (ALL_MOVEMENT_PRIMITIVE_ENVIRONMENTS, MOVEMENT_PRIMIT
 from . import envs  # noqa: F401,E402  (runs the registrations)
 from .utils.gym_compat import make, registry  # noqa: F401,E402
 from .utils.make_env_helpers import make_bb  # noqa: F401,E402
-from .vector import BlackBoxVectorEnv, make_vec  # noqa: F401,E402
+from .vector import BlackBoxVectorEnv, StepVectorEnv, make_vec  # noqa: F401,E402
 from .graph import EpisodePipeline, GraphedEpisode  # noqa: F401,E402
 
 __version__ = "0.1.0"

@@ -72,6 +72,25 @@ class FgResetIO(C.Structure):
     ]
 
 
+class FgEnvStepCfg(C.Structure):
+    _fields_ = [
+        ("struct_size", C.c_uint32),
+        ("env_kind", C.c_int32), ("n_dof", C.c_int32), ("max_episode_steps", C.c_int32), ("dt", C.c_double),
+        ("allow_self_collision", C.c_int32), ("allow_wall_collision", C.c_int32), ("collision_penalty", C.c_double),
+        ("rew_fct", C.c_int32), ("action_f64", C.c_int32),
+    ]
+
+
+class FgEnvStepIO(C.Structure):
+    _fields_ = [
+        ("struct_size", C.c_uint32),
+        ("action", C.c_void_p), ("v_is_f32", C.c_int32),
+        ("q", C.c_void_p), ("v", C.c_void_p), ("steps", C.c_void_p), ("done", C.c_void_p), ("ctx", C.c_void_p),
+        ("latch", C.c_void_p),
+        ("obs", C.c_void_p), ("reward", C.c_void_p), ("flag_bytes", C.c_void_p), ("info", C.c_void_p),
+    ]
+
+
 class FgPhaseBasis(C.Structure):
     _fields_ = [
         ("struct_size", C.c_uint32), ("phase_kind", C.c_int32), ("alpha_phase", C.c_double),
@@ -87,7 +106,7 @@ class FgPhaseBasis(C.Structure):
 # every symbol include/fancy_gym_b200.h declares (tests check the library exports all of them)
 EXPORTED_SYMBOLS = [
     "fg_last_error", "fg_abi_version", "fg_create", "fg_destroy", "fg_num_params", "fg_obs_full_dim",
-    "fg_rollout", "fg_trajgen", "fg_trajgen_phase", "fg_reset", "fg_traj_cov", "fg_traj_cov_work_floats", "fg_ffma_probe",
+    "fg_rollout", "fg_trajgen", "fg_trajgen_phase", "fg_reset", "fg_env_step", "fg_traj_cov", "fg_traj_cov_work_floats", "fg_ffma_probe",
 ]
 
 LIB_PATH = os.environ.get("FG_LIB_PATH") or os.path.join(os.path.dirname(os.path.abspath(__file__)), "lib", "libfancygym_b200.so")
@@ -127,6 +146,8 @@ def _load():
     lib.fg_traj_cov.restype = C.c_int
     lib.fg_reset.argtypes = [C.POINTER(FgResetCfg), C.POINTER(FgResetIO), C.c_int64, C.c_void_p]
     lib.fg_reset.restype = C.c_int
+    lib.fg_env_step.argtypes = [C.POINTER(FgEnvStepCfg), C.POINTER(FgEnvStepIO), C.c_int64, C.c_void_p]
+    lib.fg_env_step.restype = C.c_int
     lib.fg_ffma_probe.argtypes = [C.c_int32, C.c_int32, C.c_void_p, C.POINTER(C.c_double), C.c_void_p]
     lib.fg_ffma_probe.restype = C.c_int
     return lib

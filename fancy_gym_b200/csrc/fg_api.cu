@@ -12,6 +12,7 @@
 #include "fancy_gym_b200.h"
 #include "fg_device.cuh"
 #include "fg_dispatch.h"
+#include "fg_env_step.h"
 #include "fg_reset.cuh"
 
 namespace {
@@ -391,6 +392,37 @@ fg_status fg_reset(const fg_reset_cfg* cfg, const fg_reset_io* io, int64_t B, vo
   const cudaError_t e = cudaGetLastError();
   if (prev != cfg->device) cudaSetDevice(prev);
   if (e != cudaSuccess) return fail(FG_ERR_CUDA, "fg_reset launch: %s", cudaGetErrorString(e));
+  return FG_OK;
+}
+
+fg_status fg_env_step(const fg_env_step_cfg* cfg, const fg_env_step_io* io, int64_t B, void* stream) {
+  if (!cfg || !io) return fail(FG_ERR_INVALID, "fg_env_step: null argument");
+  if (cfg->struct_size != sizeof(fg_env_step_cfg) || io->struct_size != sizeof(fg_env_step_io))
+    return fail(FG_ERR_INVALID, "fg_env_step: struct_size mismatch (ABI)");
+  if (cfg->env_kind == FG_ENV_TOY) return fail(FG_ERR_UNSUPPORTED, "fg_env_step: the toy env has no step kernel");
+  if (cfg->env_kind < FG_ENV_HOLE_REACHER || cfg->env_kind > FG_ENV_SIMPLE_REACHER)
+    return fail(FG_ERR_INVALID, "fg_env_step: unknown env_kind %d", cfg->env_kind);
+  if (cfg->n_dof < 2 || cfg->n_dof > 7)
+    return fail(FG_ERR_UNSUPPORTED, "fg_env_step: n_dof %d outside the instantiated 2..7", cfg->n_dof);
+  if (cfg->env_kind == FG_ENV_HOLE_REACHER && (cfg->rew_fct < 0 || cfg->rew_fct > 2))
+    return fail(FG_ERR_INVALID, "fg_env_step: hole reacher rew_fct %d unknown (0 simple, 1 vel_acc, 2 unbounded)", cfg->rew_fct);
+  if (!(cfg->dt > 0.0)) return fail(FG_ERR_INVALID, "fg_env_step: dt must be positive");
+  if (B < 0) return fail(FG_ERR_INVALID, "fg_env_step: negative batch");
+  if (!io->action || !io->q || !io->v || !io->steps || !io->done || !io->ctx || !io->obs || !io->reward || !io->flag_bytes ||
+      !io->info)
+    return fail(FG_ERR_INVALID, "fg_env_step: a required buffer is NULL");
+  if (cfg->env_kind == FG_ENV_HOLE_REACHER && cfg->rew_fct == 2 && !io->latch)
+    return fail(FG_ERR_INVALID, "fg_env_step: rew_fct \"unbounded\" needs the latch buffer");
+  if (B == 0) return FG_OK;
+  fg::EnvStepDev c;
+  memset(&c, 0, sizeof(c));
+  c.dt = cfg->dt; c.dt_f = (float)cfg->dt; c.max_steps = cfg->max_episode_steps;
+  c.allow_self = cfg->allow_self_collision; c.allow_wall = cfg->allow_wall_collision; c.rew_fct = cfg->rew_fct;
+  c.penalty = cfg->collision_penalty;
+  const char* why = nullptr;
+  const cudaError_t e = fg::launch_env_step(c, cfg->env_kind, cfg->n_dof, cfg->action_f64 != 0, *io, B, (cudaStream_t)stream, &why);
+  if (why) return fail(FG_ERR_UNSUPPORTED, "fg_env_step: %s", why);
+  if (e != cudaSuccess) return fail(FG_ERR_CUDA, "fg_env_step launch: %s", cudaGetErrorString(e));
   return FG_OK;
 }
 

@@ -1,9 +1,10 @@
 """Batched step-env state holders for the classic_control reachers.
 
-The dynamics themselves run inside the fused CUDA kernel (fancy_gym_b200/csrc/fg_rollout.cuh);
-these classes own the per-env device state (joint angles / velocities / step counters / task
-context), the spaces, the constructor kwargs of the reference envs and the reset-time context
-sampling:
+The dynamics themselves run on the device: inside the fused rollout kernel for the black-box ids
+(fancy_gym_b200/csrc/fg_rollout.cuh), one control step per step() call for the step-based ids
+(fancy_gym_b200/csrc/fg_env_step.cu).  These classes own the per-env device state (joint angles /
+velocities / step counters / task context), the spaces, the constructor kwargs of the reference envs
+and the reset-time context sampling:
   HoleReacherEnv      fancy_gym/envs/classic_control/hole_reacher/hole_reacher.py
   ViaPointReacherEnv  fancy_gym/envs/classic_control/viapoint_reacher/viapoint_reacher.py
   SimpleReacherEnv    fancy_gym/envs/classic_control/simple_reacher/simple_reacher.py
@@ -68,6 +69,9 @@ class BaseReacherEnv(Env):
         self._seed_rngs = None
         self._rng_state = None            # [B, 5] uint64 PCG64 stream state of the device sampler
         self._was_reset = False
+        self._step_sets = None            # output ring of step()
+        self._latch = None                # [B, 2] end effector latched by rew_fct "unbounded" (step())
+        self._last_action_dtype = None    # dtype of the last step() action since the last full reset
 
     def _batch_or_none(self):
         return self.num_envs if self.num_envs > 1 else None
@@ -139,6 +143,7 @@ class BaseReacherEnv(Env):
         self.done.zero_()
         self._set_ctx({k: v.to(dev) for k, v in c.items()})
         self._was_reset = True
+        self._last_action_dtype = None
         return self.get_obs(), {}
 
     def _set_ctx(self, c):
@@ -201,7 +206,85 @@ class BaseReacherEnv(Env):
         stream = torch.cuda.current_stream(dev).cuda_stream
         _lib.check(_lib.lib.fg_reset(C.byref(cfg), C.byref(io), B, C.c_void_p(stream)))
         self._was_reset = True
+        if mask is None and state is None:
+            self._last_action_dtype = None
         return obs
+
+    # ---- step: one control step of every env (the step-based ids) --------------------------------
+    def _next_step_set(self):
+        """output buffers of the next step() from a ring of two: what a call returns stays valid while the next one runs"""
+        if self._step_sets is None:
+            B, n, dev = self.num_envs, self.n_links, self.device
+            self._step_sets = [dict(obs=torch.zeros(B, self.observation_space.shape[0], dtype=torch.float32, device=dev),
+                                    reward=torch.zeros(B, dtype=torch.float64, device=dev),
+                                    flags=torch.zeros(4, B, dtype=torch.bool, device=dev),
+                                    info=torch.zeros(B, 2, dtype=torch.float64, device=dev),
+                                    joints=torch.zeros(B, n, dtype=torch.float64, device=dev)) for _ in range(2)]
+            if getattr(self, "rew_fct", None) == "unbounded":
+                self._latch = torch.zeros(B, 2, dtype=torch.float64, device=dev)
+        self._step_sets.reverse()
+        return self._step_sets[0]
+
+    def step(self, action):
+        """base_reacher_direct.py:20-38 / base_reacher_torque.py:20-37 with the env's reward, for every env in ONE kernel
+        launch (fg_env_step), plus gymnasium's TimeLimit (max_episode_steps of the registration; a directly constructed env
+        never truncates).  action [B, n_links] (or [n_links] when num_envs == 1), torch tensor or numpy array, float32 or
+        float64 — the arithmetic follows the dtype as in the reference, and no clip is applied.
+        -> (obs [B, O] float32, reward [B] float64, terminated [B] bool, truncated [B] bool, infos), device tensors that
+        stay valid until the step after the next.  Envs that terminated or were truncated keep being stepped until they
+        are reset.  No device -> host copy and no synchronisation: the call can be captured in a CUDA graph."""
+        import ctypes as C
+        if not self._was_reset:
+            raise RuntimeError("Cannot call env.step() before calling env.reset()")
+        a = action if torch.is_tensor(action) else torch.as_tensor(np.ascontiguousarray(action))
+        if a.dtype not in (torch.float32, torch.float64):
+            raise TypeError(f"action dtype must be float32 or float64, got {a.dtype}")
+        B, n, dev = self.num_envs, self.n_links, self.device
+        if a.dim() == 1 and B == 1:
+            a = a[None]
+        if tuple(a.shape) != (B, n):
+            raise ValueError(f"expected an action of shape [{B}, {n}]" + (f" or [{n}]" if B == 1 else "") +
+                             f", got {tuple(a.shape)}")
+        a = a.to(dev, non_blocking=True).contiguous()
+        f64 = a.dtype == torch.float64
+        out = self._next_step_set()
+        cfg = _lib.FgEnvStepCfg()
+        cfg.struct_size = C.sizeof(_lib.FgEnvStepCfg)
+        cfg.env_kind, cfg.n_dof = self.env_kind, n
+        spec = getattr(self, "spec", None)
+        cfg.max_episode_steps = int(spec.max_episode_steps or 0) if spec is not None else 0
+        cfg.dt = float(self._dt)
+        cfg.allow_self_collision = int(bool(self.allow_self_collision))
+        cfg.allow_wall_collision = int(bool(getattr(self, "allow_wall_collision", False)))
+        cfg.collision_penalty = float(getattr(self, "collision_penalty", 0.0))
+        cfg.rew_fct = int(getattr(self, "rew_fct_code", 0))
+        cfg.action_f64 = int(f64)
+        io = _lib.FgEnvStepIO()
+        io.struct_size = C.sizeof(_lib.FgEnvStepIO)
+        io.action = a.data_ptr()
+        # every env that has stepped since the last reset holds the previous float32 action in v (envs at step 0 hold the
+        # float64 zeros of the reset; the kernel tells them apart by their step counter)
+        io.v_is_f32 = int(not f64 and self._last_action_dtype in (None, torch.float32))
+        io.q, io.v, io.steps, io.done, io.ctx = (self.q.data_ptr(), self.v.data_ptr(), self.steps.data_ptr(),
+                                                 self.done.data_ptr(), self.ctx.data_ptr())
+        if self._latch is not None:
+            io.latch = self._latch.data_ptr()
+        io.obs, io.reward, io.flag_bytes, io.info = (out["obs"].data_ptr(), out["reward"].data_ptr(),
+                                                     out["flags"].data_ptr(), out["info"].data_ptr())
+        with torch.cuda.device(dev):
+            stream = torch.cuda.current_stream(dev).cuda_stream
+            _lib.check(_lib.lib.fg_env_step(C.byref(cfg), C.byref(io), B, C.c_void_p(stream)))
+        self._last_action_dtype = a.dtype
+        terminated, truncated, success, collided = out["flags"]
+        infos: Dict[str, Any] = {}
+        if self.torque:
+            infos["reward_dist"], infos["reward_ctrl"] = out["info"][:, 0], out["info"][:, 1]
+        else:
+            infos["is_success"], infos["is_collided"] = success, collided
+            infos["end_effector"] = out["info"]
+            if self._latch is not None:          # hr_unbounded_reward.py:53-56
+                infos["joints"] = out["joints"].copy_(self.q)
+        return out["obs"], out["reward"], terminated, truncated, infos
 
     def _first_joint(self, rng, random_start):
         # base_reacher.py:81-86 (random start angle of the first joint, the arm is straight)

@@ -1,10 +1,12 @@
-"""gymnasium.vector.VectorEnv-shaped adapter over the batched black-box env (SURVEY.md §8f rank 4).
+"""gymnasium.vector.VectorEnv-shaped adapters over the batched black-box env (SURVEY.md §8f rank 4) and over the batched
+step-based env.
 
 RL libraries drive vector envs through  reset(seed=, options=) -> (obs[N, O], infos)  and
 step(actions[N, P]) -> (obs, rewards, terminations, truncations, infos)  on numpy arrays, with finished
 sub-envs reset automatically (gymnasium <= 0.29 semantics: the returned observation of a finished sub-env is the first
 one of its NEXT episode and the last one of the finished episode goes to infos["final_observation"]).  A black-box
-step is a whole episode, so every sub-env finishes on every step and the auto-reset is one extra fg_reset launch.
+step is a whole episode, so every sub-env finishes on every step and the auto-reset is one extra fg_reset launch.  A step-based
+step is one control step (fg_env_step); only the sub-envs that finished on it are reset, in one masked fg_reset launch.
 
 gymnasium itself is not a dependency; the attribute names follow its VectorEnv (num_envs, single_action_space,
 single_observation_space, action_space, observation_space, closed).
@@ -16,7 +18,7 @@ from typing import Any, Dict, Optional
 import numpy as np
 import torch
 
-from .utils.gym_compat import Box, make
+from .utils.gym_compat import Box, make, registry
 
 
 class BlackBoxVectorEnv:
@@ -66,5 +68,63 @@ class BlackBoxVectorEnv:
             self.closed = True
 
 
-def make_vec(env_id: str, num_envs: int, **kwargs) -> BlackBoxVectorEnv:
+class StepVectorEnv:
+    """The same adapter over a step-based env (`fancy/HoleReacher-v0`, ...): one step() is one control step of every
+    sub-env (fg_env_step).  Sub-envs that terminated or were truncated on a step are reset in one masked fg_reset launch,
+    each continuing its own context stream; their returned observation is the first one of the next episode and the last
+    one of the finished episode goes to infos["final_observation"] (gymnasium <= 0.29 auto-reset)."""
+
+    def __init__(self, env_id: str, num_envs: int, device="cuda:0", tensors: bool = False, **make_kwargs):
+        """tensors=True keeps everything on the device (torch tensors in, torch tensors out: no host round trip)."""
+        self.env = make(env_id, num_envs=num_envs, device=device, **make_kwargs)
+        if getattr(self.env, "context_sampler", None) != "device":
+            raise NotImplementedError("StepVectorEnv auto-resets through the device-side sampler (context_sampler='device')")
+        self.num_envs = int(num_envs)
+        self.tensors = bool(tensors)
+        self.single_action_space = Box(self.env.action_space.low, self.env.action_space.high, dtype=self.env.action_space.dtype)
+        self.single_observation_space = Box(self.env.observation_space.low, self.env.observation_space.high,
+                                            dtype=self.env.observation_space.dtype)
+        self.action_space = Box(self.single_action_space.low, self.single_action_space.high,
+                                dtype=self.single_action_space.dtype, batch=self.num_envs)
+        self.observation_space = Box(self.single_observation_space.low, self.single_observation_space.high,
+                                     dtype=self.single_observation_space.dtype, batch=self.num_envs)
+        self.closed = False
+        self.spec = self.env.spec
+
+    def _out(self, x):
+        return x if self.tensors or not torch.is_tensor(x) else x.cpu().numpy()
+
+    def reset(self, *, seed: Optional[int] = None, options: Optional[Dict[str, Any]] = None):
+        obs, info = self.env.reset(seed=seed, options=options)
+        return self._out(obs), info
+
+    def step(self, actions):
+        """actions [num_envs, n_links], float32 or float64 (numpy or torch) -> (obs, rewards, terminations, truncations,
+        infos)"""
+        a = actions if torch.is_tensor(actions) else torch.as_tensor(np.ascontiguousarray(actions))
+        if a.dim() == 1:
+            a = a[None]
+        obs, rew, terminated, truncated, infos = self.env.step(a)
+        infos = dict(infos)
+        infos["final_observation"] = obs
+        infos["_final_observation"] = terminated | truncated
+        # the kernel has set done = terminated | truncated: exactly the envs to reset, the others keep their rows
+        next_obs = obs.clone()
+        self.env.device_reset(None, out=next_obs, mask=self.env.done)
+        return (self._out(next_obs), self._out(rew), self._out(terminated), self._out(truncated),
+                {k: self._out(v) for k, v in infos.items()})
+
+    def close(self):
+        if not self.closed:
+            self.env.close()
+            self.closed = True
+
+
+def make_vec(env_id: str, num_envs: int, **kwargs):
+    """BlackBoxVectorEnv for a black-box id (`fancy_ProMP/HoleReacher-v0`), StepVectorEnv for a step-based one
+    (`fancy/HoleReacher-v0`)."""
+    from .envs.registry import bb_env_constructor
+    spec = registry.get(env_id)
+    if spec is not None and spec.entry_point is not bb_env_constructor:
+        return StepVectorEnv(env_id, num_envs, **kwargs)
     return BlackBoxVectorEnv(env_id, num_envs, **kwargs)

@@ -233,6 +233,40 @@ typedef struct fg_reset_io {
   float* obs;                  /* [B, n_obs_out] observation of the reset state, or NULL */
 } fg_reset_io;
 
+/* One control step of the step-based reachers (the `fancy/<Name>-v0` ids: env.step(action) as PPO / SAC call it). */
+typedef struct fg_env_step_cfg {
+  uint32_t struct_size;
+  int32_t env_kind;            /* FG_ENV_HOLE_REACHER / _VIAPOINT_REACHER / _SIMPLE_REACHER */
+  int32_t n_dof;               /* 2..7 */
+  int32_t max_episode_steps;   /* gymnasium TimeLimit: truncated = steps >= max_episode_steps; <= 0: never truncates */
+  double dt;                   /* env.dt (0.01) */
+  int32_t allow_self_collision;
+  int32_t allow_wall_collision;
+  double collision_penalty;
+  int32_t rew_fct;             /* hole reacher: 0 simple, 1 vel_acc, 2 unbounded (as fg_config) */
+  int32_t action_f64;          /* 0: action is float32 [B, dof], 1: float64 (the reference's arithmetic follows the dtype) */
+} fg_env_step_cfg;
+
+typedef struct fg_env_step_io {
+  uint32_t struct_size;
+  const void* action;          /* [B, dof] float32 or float64 (cfg.action_f64); the env applies no clip */
+  int32_t v_is_f32;            /* velocity-controlled envs: 1 if every env with steps > 0 holds the previous call's float32
+                                  action in v (then acc = (a - v) / dt is float32 arithmetic), 0 otherwise */
+  /* state, in/out (as fg_rollout_io; fg_reset writes it) */
+  double* q;                   /* [B, dof] */
+  double* v;                   /* [B, dof] */
+  int32_t* steps;              /* [B] */
+  uint8_t* done;               /* [B] out: terminated or truncated on this step */
+  const double* ctx;           /* [B, 4] */
+  double* latch;               /* [B, 2] hole reacher rew_fct "unbounded": end effector latched at step 180 or on a collision;
+                                  written before it is read within an episode (no reset needed); NULL for the other envs */
+  /* outputs */
+  float* obs;                  /* [B, n_obs_full] full step observation (3*dof + 4 / 5 / 3 columns) */
+  double* reward;              /* [B] */
+  uint8_t* flag_bytes;         /* [4, B] rows terminated, truncated, is_success, is_collided (0 / 1) */
+  double* info;                /* [B, 2] hole / viapoint: end effector x, y; simple: reward_dist, reward_ctrl */
+} fg_env_step_io;
+
 typedef struct fg_handle fg_handle;
 
 const char* fg_last_error(void);
@@ -329,6 +363,15 @@ fg_status fg_traj_cov(const fg_handle* h, const float* params_L, float reg, int3
  * reset with seed_i), zeroes velocities / step counters / done flags and writes the context observation.
  */
 fg_status fg_reset(const fg_reset_cfg* cfg, const fg_reset_io* io, int64_t B, void* stream);
+
+/*
+ * Advances B step-based envs by ONE control step — replaces env.step(action) of base_reacher_direct.py:20-38 /
+ * base_reacher_torque.py:20-37 with the reward of the configured env, plus gymnasium's TimeLimit truncation.
+ * Envs that terminated or were truncated keep being stepped (an env that is not reset keeps integrating).  Launches on
+ * the CURRENT device, on `stream`; no allocation, no synchronisation.  FG_ERR_UNSUPPORTED for the toy env and for n_dof
+ * outside 2..7.
+ */
+fg_status fg_env_step(const fg_env_step_cfg* cfg, const fg_env_step_io* io, int64_t B, void* stream);
 
 /*
  * FP32 FFMA-chain microbenchmark used as the roofline denominator of the fused rollout
