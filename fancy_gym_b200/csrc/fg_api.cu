@@ -97,8 +97,10 @@ fg_status fg_create(const fg_config* cfg, int32_t device, fg_handle** out) {
   fg::DevCfg& d = h->dev;
   memset(&d, 0, sizeof(d));
   const int T = cfg->n_steps, K = cfg->n_basis, N = cfg->n_dof;
-  d.n_dof = N; d.T = T; d.K = K; d.max_steps = cfg->max_episode_steps;
-  d.dt = cfg->dt; d.dt_f = (float)cfg->dt;
+  d.n_dof = N; d.T = T; d.K = K;
+  d.env.dt = cfg->dt; d.env.dt_f = (float)cfg->dt; d.env.max_steps = cfg->max_episode_steps;
+  d.env.allow_self = cfg->allow_self_collision; d.env.allow_wall = cfg->allow_wall_collision;
+  d.env.rew_fct = cfg->rew_fct; d.env.wall_mode = cfg->wall_mode; d.env.penalty = cfg->collision_penalty;
   const bool torque = cfg->env_kind == FG_ENV_SIMPLE_REACHER;
   // Box(low=-bound, high=bound) with the default float32 dtype (base_reacher_direct.py:16-18, _torque.py:16-18;
   // ToyEnv: +-1, test_black_box.py:29)
@@ -106,13 +108,9 @@ fg_status fg_create(const fg_config* cfg, int32_t device, fg_handle** out) {
   for (int i = 0; i < FG_MAX_DOF; ++i) { d.p[i] = cfg->p_gains[i]; d.d[i] = cfg->d_gains[i]; }
   d.tau = cfg->tau; d.alpha = cfg->dmp_alpha; d.beta = cfg->dmp_alpha / 4.0f;
   d.wscale = cfg->weights_scale; d.gscale = cfg->goal_scale; d.rel_goal = cfg->relative_goal;
-  d.allow_self = cfg->allow_self_collision; d.allow_wall = cfg->allow_wall_collision;
-  d.rew_fct = cfg->rew_fct; d.wall_mode = cfg->wall_mode; d.time_aware = cfg->time_aware; d.ctrl = cfg->ctrl_kind;
-  d.penalty = cfg->collision_penalty;
+  d.time_aware = cfg->time_aware; d.ctrl = cfg->ctrl_kind;
   d.n_obs_out = cfg->n_obs_out;
-  const int extra[4] = {4, 5, 3, -2};   // hole: width, ee-goal(2), steps; viapoint: 2+2+1; simple: 2+1; toy: obs dim 1
-  d.n_obs_full = 3 * N + extra[cfg->env_kind] + (cfg->time_aware ? 1 : 0);
-  if (cfg->env_kind == FG_ENV_TOY) d.n_obs_full = 1 + (cfg->time_aware ? 1 : 0);
+  d.n_obs_full = fg::obs_dim(cfg->env_kind, N) + (cfg->time_aware ? 1 : 0);
   for (int j = 0; j < cfg->n_obs_out; ++j) {
     if (cfg->obs_index[j] < 0 || cfg->obs_index[j] >= d.n_obs_full) {
       cudaSetDevice(prev);
@@ -368,8 +366,7 @@ fg_status fg_reset(const fg_reset_cfg* cfg, const fg_reset_io* io, int64_t B, vo
     return fail(FG_ERR_INVALID, "fg_reset: env_kind %d has no reset sampler", cfg->env_kind);
   if (cfg->n_dof < 1 || cfg->n_dof > FG_MAX_DOF) return fail(FG_ERR_INVALID, "fg_reset: n_dof %d out of range", cfg->n_dof);
   if (cfg->n_obs_out < 0 || cfg->n_obs_out > FG_MAX_OBS) return fail(FG_ERR_INVALID, "fg_reset: n_obs_out out of range");
-  const int extra[3] = {4, 5, 3};
-  const int n_full = 3 * cfg->n_dof + extra[cfg->env_kind] + (cfg->time_aware ? 1 : 0);
+  const int n_full = fg::obs_dim(cfg->env_kind, cfg->n_dof) + (cfg->time_aware ? 1 : 0);
   for (int j = 0; j < cfg->n_obs_out; ++j)
     if (cfg->obs_index[j] < 0 || cfg->obs_index[j] >= n_full)
       return fail(FG_ERR_INVALID, "fg_reset: obs_index[%d]=%d outside the %d-wide observation", j, cfg->obs_index[j], n_full);
@@ -414,7 +411,7 @@ fg_status fg_env_step(const fg_env_step_cfg* cfg, const fg_env_step_io* io, int6
   if (cfg->env_kind == FG_ENV_HOLE_REACHER && cfg->rew_fct == 2 && !io->latch)
     return fail(FG_ERR_INVALID, "fg_env_step: rew_fct \"unbounded\" needs the latch buffer");
   if (B == 0) return FG_OK;
-  fg::EnvStepDev c;
+  fg::ReacherCfg c;
   memset(&c, 0, sizeof(c));
   c.dt = cfg->dt; c.dt_f = (float)cfg->dt; c.max_steps = cfg->max_episode_steps;
   c.allow_self = cfg->allow_self_collision; c.allow_wall = cfg->allow_wall_collision; c.rew_fct = cfg->rew_fct;

@@ -22,16 +22,23 @@ namespace fg {
 constexpr double kPi = 3.141592653589793115997963468544185161590576171875;   // numpy.pi
 constexpr int kLinePoints = 100;                                             // hole_reacher.py:149
 
-// Kernel-side copy of fg_config (passed by value as a __grid_constant__ kernel parameter).
-struct DevCfg {
-  int n_dof, T, K, max_steps;
+// The settings of one reacher env step (fg_reacher.cuh), filled from fg_config or fg_env_step_cfg.
+struct ReacherCfg {
   double dt;        // python float 0.01
   float dt_f;       // float32(0.01): numpy's weak-scalar promotion when the action is float32
+  int max_steps;    // <= 0: never truncates (fg_env_step)
+  int allow_self, allow_wall, rew_fct, wall_mode;
+  double penalty;
+};
+
+// Kernel-side copy of fg_config (passed by value as a __grid_constant__ kernel parameter).
+struct DevCfg {
+  int n_dof, T, K;
+  ReacherCfg env;
   float act_lim;    // action-space bound as float32 (2*pi or 1000)
   double p[FG_MAX_DOF], d[FG_MAX_DOF];
   float tau, alpha, beta, wscale, gscale;
-  int rel_goal, allow_self, allow_wall, rew_fct, wall_mode, time_aware, ctrl;
-  double penalty;
+  int rel_goal, time_aware, ctrl;
   int n_obs_out, n_obs_full;
   int obs_index[FG_MAX_OBS];
   const float* tab_a;   // device

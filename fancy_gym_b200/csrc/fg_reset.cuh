@@ -7,7 +7,7 @@
 // numpy algorithms restated (numpy/random/bit_generator.pyx, src/pcg64/pcg64.h, src/distributions/distributions.c):
 // see oracle/np_rng.py, which is pinned against numpy and is the specification of this file.
 #pragma once
-#include "fg_device.cuh"
+#include "fg_reacher.cuh"
 
 namespace fg {
 
@@ -200,19 +200,7 @@ k_reset(const __grid_constant__ ResetCfg c, const __grid_constant__ fg_reset_io 
     obs[2 * N + i] = 0.0f;
   }
   int no = 3 * N;
-  if (c.env_kind == FG_ENV_HOLE_REACHER) {
-    obs[no++] = (float)ctx[1];
-    obs[no++] = (float)(ex - ctx[0]);
-    obs[no++] = (float)(ey - (-ctx[2]));
-  } else if (c.env_kind == FG_ENV_VIAPOINT_REACHER) {
-    obs[no++] = (float)(ex - ctx[0]);
-    obs[no++] = (float)(ey - ctx[1]);
-    obs[no++] = (float)(ex - ctx[2]);
-    obs[no++] = (float)(ey - ctx[3]);
-  } else {
-    obs[no++] = (float)(ex - ctx[0]);
-    obs[no++] = (float)(ey - ctx[1]);
-  }
+  no += obs_tail(c.env_kind, ctx, ex, ey, obs + no);
   obs[no++] = 0.0f;                       // steps
   if (c.time_aware) obs[no++] = 0.0f;     // elapsed / max_episode_steps
   if (io.obs)

@@ -19,7 +19,7 @@
 #ifdef FG_ROLLOUT_CHECK
 #include <cstdio>
 #endif
-#include "fg_device.cuh"
+#include "fg_reacher.cuh"
 
 namespace fg {
 
@@ -154,8 +154,7 @@ k_rollout(const __grid_constant__ DevCfg c, const __grid_constant__ fg_rollout_i
   }
   if constexpr (MP == FG_MP_PROMP)
     for (int i = tid; i < c.rows_b; i += BD) tabR[i] = __frcp_rn(c.tab_b[i]);
-  for (int i = tid; i < kLinePoints; i += BD)   // float32(numpy.linspace(0,1,100)): i*(1/99) in float64, last forced to 1
-    s_m[i] = (i == kLinePoints - 1) ? 1.0f : (float)((double)i * (1.0 / 99.0));
+  stage_line_points<BD>(s_m);
 
   // Envs per block: `warps_lo` warps, one more in the first `blocks_extra` blocks (the launcher uses full blocks: 4 / 0).
   const int bi = (int)blockIdx.x;
@@ -201,7 +200,7 @@ k_rollout(const __grid_constant__ DevCfg c, const __grid_constant__ fg_rollout_i
   float carry_a[N], carry_b[N];     // ProMP: pos[t+1], vel[t]; DMP: y, scaled-time velocity
   float pos[N], vel[N];             // desired position / velocity of the current step
   Hole hole{};
-  double cx0 = 0, cx1 = 0, cx2 = 0, cx3 = 0;
+  double cx[4] = {0, 0, 0, 0};
   // rew_fct "unbounded": the end effector latched at step 180 (hr_unbounded_reward.py:35-36) lives in the env's slot, not in
   // registers (it is touched on two steps of an episode)
   auto latch_put = [&](double x, double y) {
@@ -249,8 +248,8 @@ k_rollout(const __grid_constant__ DevCfg c, const __grid_constant__ fg_rollout_i
   auto weight = [&](int d, int kk) -> float {
     if constexpr (KC > 0) return wreg[d][kk]; else return WSM(d, kk);
   };
-  const float r_tau = __frcp_rn(c.tau), r_dt = __frcp_rn(c.dt_f);
-  const double r_dt64 = __drcp_rn(c.dt);
+  const float r_tau = __frcp_rn(c.tau), r_dt = __frcp_rn(c.env.dt_f);
+  const double r_dt64 = __drcp_rn(c.env.dt);
 
   // ---- per-env phase (NTX > 0): this env's tau / delay / time grid, and the basis row of one time point -----------------
   float tau_b = c.tau, delay_b = 0.f, r_tau_b = r_tau;
@@ -322,13 +321,9 @@ k_rollout(const __grid_constant__ DevCfg c, const __grid_constant__ fg_rollout_i
   // ---- the env's context (read again whenever a thread picks an env up: a few L2 hits per re-packing) ----
   auto load_context = [&]() {
     if constexpr (ENV != FG_ENV_TOY) {
-      cx0 = io.ctx[b * 4 + 0]; cx1 = io.ctx[b * 4 + 1]; cx2 = io.ctx[b * 4 + 2]; cx3 = io.ctx[b * 4 + 3];
+      cx[0] = io.ctx[b * 4 + 0]; cx[1] = io.ctx[b * 4 + 1]; cx[2] = io.ctx[b * 4 + 2]; cx[3] = io.ctx[b * 4 + 3];
     }
-    if constexpr (ENV == FG_ENV_HOLE_REACHER) {
-      hole.xl = (float)(cx0 - cx1 / 2);    // hole_reacher.py:152 (x - width/2), rounded once to float32
-      hole.xr = (float)(cx0 + cx1 / 2);
-      hole.nd = (float)(-cx2);
-    }
+    if constexpr (ENV == FG_ENV_HOLE_REACHER) hole = hole_of(cx);
   };
   auto plan_seg = [&](int kk) -> int {       // steps plan kk may execute (ragged sub-trajectories: per env)
     if (io.n_plans > 1) return io.plan_seg[kk];
@@ -367,32 +362,10 @@ k_rollout(const __grid_constant__ DevCfg c, const __grid_constant__ fg_rollout_i
   // full step observation (float64 trig, cast to float32 like _get_obs) given the end effector; returns its width
   auto build_obs = [&](float* obs, double ex, double ey) -> int {
     int no = 0;
-    if constexpr (ENV == FG_ENV_TOY) {
-      obs[no++] = -1.0f;
-    } else {
-#pragma unroll
-      for (int i = 0; i < N; ++i) obs[i] = (float)cos(q[i]);
-#pragma unroll
-      for (int i = 0; i < N; ++i) obs[N + i] = (float)sin(q[i]);
-#pragma unroll
-      for (int i = 0; i < N; ++i) obs[2 * N + i] = VF ? vf[i] : (float)v[i];
-      no = 3 * N;
-      if constexpr (ENV == FG_ENV_HOLE_REACHER) {
-        obs[no++] = (float)cx1;
-        obs[no++] = (float)(ex - cx0);
-        obs[no++] = (float)(ey - (-cx2));
-      } else if constexpr (ENV == FG_ENV_VIAPOINT_REACHER) {
-        obs[no++] = (float)(ex - cx0);
-        obs[no++] = (float)(ey - cx1);
-        obs[no++] = (float)(ex - cx2);
-        obs[no++] = (float)(ey - cx3);
-      } else {
-        obs[no++] = (float)(ex - cx0);
-        obs[no++] = (float)(ey - cx1);
-      }
-      obs[no++] = (float)steps;
-    }
-    if (c.time_aware) obs[no++] = (float)((double)steps / (double)c.max_steps);
+    if constexpr (ENV == FG_ENV_TOY) obs[no++] = -1.0f;
+    else if constexpr (VF) no = reacher_obs<ENV, N>(obs, q, vf, cx, ex, ey, steps);
+    else no = reacher_obs<ENV, N>(obs, q, v, cx, ex, ey, steps);
+    if (c.time_aware) obs[no++] = (float)((double)steps / (double)c.env.max_steps);
     return no;
   };
   auto end_effector_now = [&](double& ex, double& ey) {
@@ -556,24 +529,7 @@ k_rollout(const __grid_constant__ DevCfg c, const __grid_constant__ fg_rollout_i
     end_effector_now(ex, ey);
     if (fl & kSlotDeferred) {
       // the reward of the step that collided (its distance term needs the float64 end effector): the last addend of the return
-      double reward = 0.0;
-      if constexpr (ENV == FG_ENV_HOLE_REACHER) {
-        if (c.rew_fct == 0) {          // hr_simple_reward.py:35-53 with collision_cost = 1
-          const double dx = ex - cx0, dy = ey - (-cx2);
-          const double dist = sqrt(dx * dx + dy * dy);
-          reward = __dadd_rn(__dadd_rn(__dmul_rn(dist * dist, -1.0), aux), __dmul_rn(1.0, -c.penalty));
-        } else {                       // hr_unbounded_reward.py: the end effector is latched on the collision
-          latch_put(ex, ey);
-          const double dx = ex - cx0, dy = ey - (-cx2);
-          const double dist = sqrt(dx * dx + dy * dy);
-          reward = __dadd_rn(0.25 * exp(-dist), __dmul_rn(aux, -5e-6));
-        }
-      } else if constexpr (ENV == FG_ENV_VIAPOINT_REACHER) {      // viapoint_reacher.py:96-101
-        const double dist = sqrt((ex - cx2) * (ex - cx2) + (ey - cx3) * (ey - cx3));
-        reward = -c.penalty;
-        reward -= dist * dist;
-        reward -= aux;
-      }
+      const double reward = collided_reward<ENV>(c.env, cx, aux, ex, ey, latch_put);
       ret += reward;
       if constexpr (DBG) {
         if (io.dbg_rewards) io.dbg_rewards[b * c.T + tl - 1] = reward;
@@ -650,7 +606,7 @@ k_rollout(const __grid_constant__ DevCfg c, const __grid_constant__ fg_rollout_i
     ret = 0.0;
     load_context();
     if constexpr (ENV == FG_ENV_HOLE_REACHER) {
-      if (c.rew_fct == 2 && steps > 0) latch_put(io.info[b * 4 + 2], io.info[b * 4 + 3]);   // a later plan segment of the episode
+      if (c.env.rew_fct == 2 && steps > 0) latch_put(io.info[b * 4 + 2], io.info[b * 4 + 3]);   // a later plan segment of the episode
       else latch_put(0.0, 0.0);
     }
     float ybc[N], vbc[N];
@@ -785,7 +741,6 @@ k_rollout(const __grid_constant__ DevCfg c, const __grid_constant__ fg_rollout_i
         // ---------------------------------------------------------------- controller + clip + dynamics
         double a64[N];
         float a32[N];
-        double acc_cost = 0.0;    // sum(acc^2) (direct envs), in the reference's dtype
         if constexpr (MOTOR) {    // pd_controller.py:28: float64 because c_pos / c_vel are float64
 #pragma unroll
           for (int i = 0; i < N; ++i) {
@@ -804,36 +759,10 @@ k_rollout(const __grid_constant__ DevCfg c, const __grid_constant__ fg_rollout_i
           }
         }
 
-        if constexpr (ENV == FG_ENV_HOLE_REACHER || ENV == FG_ENV_VIAPOINT_REACHER) {
-          // base_reacher_direct.py:25-27
-          if (MOTOR || steps == 0) {      // v is float64 (zeros at reset / float64 actions): float64 arithmetic
-#pragma unroll
-            for (int i = 0; i < N; ++i) {
-              const double ac = div_by64(a64[i] - (VF ? (double)vf[i] : v[i]), c.dt, r_dt64);
-              acc_cost += ac * ac;
-            }
-          } else {                        // float32 action and float32 velocity
-            float s32 = 0.f;
-#pragma unroll
-            for (int i = 0; i < N; ++i) {
-              const float ac = div_by(__fsub_rn(a32[i], VF ? vf[i] : (float)v[i]), c.dt_f, r_dt);
-              s32 = __fadd_rn(s32, __fmul_rn(ac, ac));
-            }
-            acc_cost = (double)s32;
-          }
-#pragma unroll
-          for (int i = 0; i < N; ++i) {
-            if constexpr (VF) vf[i] = a32[i]; else v[i] = a64[i];
-            q[i] += MOTOR ? __dmul_rn(c.dt, a64[i]) : (double)__fmul_rn(c.dt_f, a32[i]);
-          }
-        } else if constexpr (ENV == FG_ENV_SIMPLE_REACHER) {
-          // base_reacher_torque.py:25-26
-#pragma unroll
-          for (int i = 0; i < N; ++i) {
-            v[i] += MOTOR ? __dmul_rn(c.dt, a64[i]) : (double)__fmul_rn(c.dt_f, a32[i]);
-            q[i] += __dmul_rn(c.dt, v[i]);
-          }
-        }
+        // v is float64 (zeros at reset / float64 actions) unless it holds the previous float32 action
+        double acc_cost;
+        if constexpr (VF) acc_cost = reacher_dynamics<ENV, N, MOTOR>(c.env, r_dt, r_dt64, q, vf, a64, a32, MOTOR || steps == 0);
+        else acc_cost = reacher_dynamics<ENV, N, MOTOR>(c.env, r_dt, r_dt64, q, v, a64, a32, MOTOR || steps == 0);
 
         // ---------------------------------------------------------------- geometry, collisions, reward
         double reward = 0.0;
@@ -846,154 +775,24 @@ k_rollout(const __grid_constant__ DevCfg c, const __grid_constant__ fg_rollout_i
           th[0] = q[0];
 #pragma unroll
           for (int i = 1; i < N; ++i) th[i] = th[i - 1] + q[i];
-
-          if constexpr (ENV == FG_ENV_HOLE_REACHER) {
-            float cs[N], sn[N];
-#pragma unroll
-            for (int i = 0; i < N; ++i) sincos_reduced(th[i], sn[i], cs[i]);
-            bool selfc = false, wallc = false;
-            if (!c.allow_self) selfc = self_collision<N>(q, th, cs, sn);
-            if (!c.allow_wall) wallc = wall_collision<N>(s_m, cs, sn, hole, c.wall_mode);
-            collided = selfc | wallc;
-            if (c.rew_fct == 0) {
-              // hr_simple_reward.py:35-53
-              // ordinary steps: (-0.0 + x) + -0.0 == x for x = acc_cost * -5e-8 <= 0, so only the product is formed
-              reward = __dmul_rn(acc_cost, -5e-8);
-              if (collided) {           // the distance term is added when the env is finished (see finish())
-                deferred = true;
-                defer(reward);
-                reward = 0.0;
-              } else if (steps == 199) {
-                double ex, ey;
-                end_effector64<N>(th, ex, ey);
-                const double dx = ex - cx0, dy = ey - (-cx2);
-                const double dist = sqrt(dx * dx + dy * dy);
-                const double dist_cost = dist * dist;
-                success = dist < 0.005;
-                reward = __dadd_rn(__dadd_rn(__dmul_rn(dist_cost, -1.0), reward), __dmul_rn(0.0, -c.penalty));
-              }
-            } else if (c.rew_fct == 1) {
-              // hr_dist_vel_acc_reward.py:20-60: distance / collision terms only on step 199 (a collision ends the episode, so
-              // the latched flag and collision_dist are this step's); factors (-1, -1e-4, -1e-6, -penalty, 0)
-              double dist_cost = 0.0, coll_cost = 0.0;
-              if (steps == 199) {
-                double ex, ey;
-                end_effector64<N>(th, ex, ey);
-                const double dx = ex - cx0, dy = ey - (-cx2);
-                const double dist = sqrt(dx * dx + dy * dy);
-                dist_cost = dist * dist;
-                coll_cost = collided ? dist * dist : 0.0;
-                success = (dist < 0.005) && !collided;
-              }
-              double vel_cost;
-              if constexpr (MOTOR) {
-                vel_cost = 0.0;
-#pragma unroll
-                for (int i = 0; i < N; ++i) vel_cost += a64[i] * a64[i];
-              } else {      // float32 action: np.sum(v ** 2) is a float32 sum
-                float s32 = 0.f;
-#pragma unroll
-                for (int i = 0; i < N; ++i) s32 = __fadd_rn(s32, __fmul_rn(a32[i], a32[i]));
-                vel_cost = (double)s32;
-              }
-              reward = __dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(dist_cost, -1.0), __dmul_rn(vel_cost, -1e-4)),
-                                           __dmul_rn(acc_cost, -1e-6)), __dmul_rn(coll_cost, -c.penalty));
-            } else {
-              // hr_unbounded_reward.py:17-60: end effector latched at step 180 (or on collision); factors (1, -5e-6)
-              if (collided) {           // latch + distance reward when the env is finished (see finish())
-                deferred = true;
-                defer(acc_cost);
-              } else {
-                double dist_reward = 0.0;
-                if (steps == 180 || steps == 199) {
-                  double ex, ey;
-                  end_effector64<N>(th, ex, ey);
-                  if (steps == 180) {
-                    latch_put(ex, ey);
-                  }
-                  if (steps == 199) {
-                    double ee180x, ee180y;
-                    latch_get(ee180x, ee180y);
-                    const double dx = ee180x - cx0, dy = ee180y - (-cx2);
-                    const double dist = sqrt(dx * dx + dy * dy);
-                    if (ey > 0) dist_reward = exp(-dist);
-                    else dist_reward = 1 - ee180y;
-                    success = true;
-                  }
-                }
-                reward = __dadd_rn(dist_reward, __dmul_rn(acc_cost, -5e-6));
-              }
-            }
+          // the float64 end effector only on the steps whose reward reports it
+          const StepReward r = reacher_reward<ENV, N, MOTOR>(c.env, q, th, a64, a32, acc_cost, steps, cx, hole, s_m,
+                                                             [&](double& ex, double& ey) { end_effector64<N>(th, ex, ey); },
+                                                             latch_get, latch_put);
+          reward = r.reward;
+          collided = r.collided;
+          success = r.success;
+          deferred = r.deferred;
+          if (deferred) defer(r.aux);   // the rest of this reward is added when the env is finished (see finish())
+          if constexpr (ENV == FG_ENV_SIMPLE_REACHER) {
+            info0 = r.info0;
+            info1 = r.info1;
+          } else {
             terminated = collided;
-          } else if constexpr (ENV == FG_ENV_VIAPOINT_REACHER) {
-            // viapoint_reacher.py:79-107 (App. A.6-Q1/Q2: -inf start, `acc` is the action)
-            if (!c.allow_self) {
-              collided = joint_limits<N>(q);
-#ifndef FG_VIAPOINT_SCREEN
-#define FG_VIAPOINT_SCREEN 1
-#endif
-              if (!FG_VIAPOINT_SCREEN || may_self_intersect<N>(q)) {      // (the link directions are only needed for the pair tests)
-                float cs[N], sn[N];
-#pragma unroll
-                for (int i = 0; i < N; ++i) sincos_reduced(th[i], sn[i], cs[i]);
-                collided |= links_intersect<N>(th, cs, sn);
-              }
-            }
-            double act_term;
-            if constexpr (MOTOR) {
-              double asq = 0.0;
-#pragma unroll
-              for (int i = 0; i < N; ++i) asq += a64[i] * a64[i];
-              act_term = 5e-8 * asq;
-            } else {   // float32 action: np.sum(acc**2) is float32 and 5e-8 * float32 stays float32
-              float s32 = 0.f;
-#pragma unroll
-              for (int i = 0; i < N; ++i) s32 = __fadd_rn(s32, __fmul_rn(a32[i], a32[i]));
-              act_term = (double)__fmul_rn(5e-8f, s32);
-            }
-            if (!collided) {
-              double dist = INFINITY;
-              reward = -INFINITY;
-              if (steps == 100 || steps == 199) {
-                double ex, ey;
-                end_effector64<N>(th, ex, ey);
-                const double tx = (steps == 100) ? cx0 : cx2, ty = (steps == 100) ? cx1 : cx3;
-                dist = sqrt((ex - tx) * (ex - tx) + (ey - ty) * (ey - ty));
-              }
-              success = dist < 0.005;
-              reward -= dist * dist;
-              reward -= act_term;
-            } else {                    // -penalty - dist^2 - act_term when the env is finished (see finish())
-              deferred = true;
-              defer(act_term);
-            }
-            terminated = collided;
-          } else {   // SIMPLE_REACHER: simple_reacher.py:56-70 (collision flag is computed but unused)
-            double rdist = 0.0;
-            if (steps >= 199) {
-              double ex, ey;
-              end_effector64<N>(th, ex, ey);
-              rdist = -sqrt((ex - cx0) * (ex - cx0) + (ey - cx1) * (ey - cx1));
-            }
-            double rctrl;
-            if constexpr (MOTOR) {
-              rctrl = 0.0;
-#pragma unroll
-              for (int i = 0; i < N; ++i) rctrl += a64[i] * a64[i];
-              reward = rdist - rctrl;
-            } else {   // float32 action: reward_ctrl float32; `0 - float32` stays float32 before steps>=199
-              float s32 = 0.f;
-#pragma unroll
-              for (int i = 0; i < N; ++i) s32 = __fadd_rn(s32, __fmul_rn(a32[i], a32[i]));
-              rctrl = (double)s32;
-              reward = (steps >= 199) ? rdist - rctrl : (double)(0.f - s32);
-            }
-            info0 = rdist;
-            info1 = rctrl;
           }
         }
         steps += 1;
-        const bool truncated = steps >= c.max_steps;       // gymnasium TimeLimit (App. A.6-Q12)
+        const bool truncated = steps >= c.env.max_steps;       // gymnasium TimeLimit (App. A.6-Q12)
         ret += reward;            // (+0.0 for a deferred step: the return is never -0.0, so this leaves it as it is)
 
         if constexpr (DBG) {
