@@ -101,6 +101,11 @@ class MPInterface:
         onto the parameters, mp/assumptions.py)"""
         return local
 
+    def _param_scale(self, device):
+        """hook: float32 factors [params per dof] that multiply the parameters because the switch scale_on_library_side
+        moved the scales off the basis table; None while the scales sit on the table"""
+        return None
+
     def boundary_prestep(self, params, pos, vel):
         """hook: boundary condition the kernels should start from instead of (pos, vel); None = as given"""
         return None
@@ -292,14 +297,20 @@ class MPInterface:
         D = self._num_local_params
         if L.shape[1:] != (D, D):
             raise ValueError(f"params_L must be [.., {D}, {D}], got {tuple(L.shape)}")
+        s = self._param_scale(L.device)
+        if s is not None:
+            # the kernels read the basis table, which then lacks the scales: the trajectories are Psi (S w), so their
+            # covariance is Psi (S L)(S L)^T Psi^T; scaling rows keeps L lower triangular
+            L = (L.view(B, N, D // N, D) * s[:, None]).view(B, D, D)
         h = self._trajgen_handle()
         cov = torch.empty(B, N * T, N * T, device=self.device, dtype=torch.float32) if want_cov else None
         std = torch.empty(B, T, N, device=self.device, dtype=torch.float32) if want_std else None
-        work = torch.empty(int(_lib.lib.fg_traj_cov_work_floats(h, B)), device=self.device, dtype=torch.float32)
-        stream = torch.cuda.current_stream(self.device).cuda_stream
-        _lib.check(_lib.lib.fg_traj_cov(h, L.data_ptr(), float(reg), int(bool(batch_scope)),
-                                        cov.data_ptr() if want_cov else None, std.data_ptr() if want_std else None,
-                                        work.data_ptr(), int(path), B, C.c_void_p(stream)))
+        if B > 0:       # (empty tensors have null data pointers, which fg_traj_cov refuses)
+            work = torch.empty(int(_lib.lib.fg_traj_cov_work_floats(h, B)), device=self.device, dtype=torch.float32)
+            stream = torch.cuda.current_stream(self.device).cuda_stream
+            _lib.check(_lib.lib.fg_traj_cov(h, L.data_ptr(), float(reg), int(bool(batch_scope)),
+                                            cov.data_ptr() if want_cov else None, std.data_ptr() if want_std else None,
+                                            work.data_ptr(), int(path), B, C.c_void_p(stream)))
         if not batched:
             cov, std = (cov[0] if want_cov else None), (std[0] if want_std else None)
         return cov, std
@@ -343,6 +354,11 @@ class ProMP(MPInterface):
         if not self.phase_gn.assume["scale_on_library_side"]:       # the scale sits on the parameters (one float32 multiply)
             local = local.to(torch.float32) * float(np.float32(self.weights_scale))
         return local
+
+    def _param_scale(self, device):
+        if self.phase_gn.assume["scale_on_library_side"]:
+            return None
+        return torch.full((self.basis_gn.num_basis,), float(np.float32(self.weights_scale)), dtype=torch.float32, device=device)
 
     def tables(self) -> MPTables:
         t32 = self.times32()
@@ -473,9 +489,7 @@ class ProDMP(MPInterface):
         v = local.view(*local.shape[:-1], self.num_dof, K + 1)
         gs = float(self.goal_scale)
         if not on_basis:
-            sc = torch.full((K + 1,), float(np.float32(self.weights_scale)), dtype=torch.float32, device=local.device)
-            sc[K] = float(np.float32(gs))
-            v *= sc
+            v *= self._param_scale(local.device)
         if self.goal_offset:
             if A["goal_offset_after_scale"]:
                 off = self.goal_offset / gs if on_basis else self.goal_offset
@@ -483,6 +497,14 @@ class ProDMP(MPInterface):
                 off = self.goal_offset if on_basis else self.goal_offset * gs
             v[..., -1] += float(np.float32(off))
         return local
+
+    def _param_scale(self, device):
+        if self.phase_gn.assume["scale_on_library_side"]:
+            return None
+        K = self.basis_gn.num_basis
+        sc = torch.full((K + 1,), float(np.float32(self.weights_scale)), dtype=torch.float32, device=device)
+        sc[K] = float(np.float32(self.goal_scale))
+        return sc
 
     def tables(self) -> MPTables:
         bg = self.basis_gn

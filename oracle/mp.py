@@ -511,6 +511,12 @@ class ProMP(MPBase):
         z0 = getattr(bg, "num_basis_zero_start", 0)
         return b[..., z0:z0 + bg.num_basis]
 
+    def cov_basis(self):
+        """[T, Kc] basis of traj_pos_cov: weights_scale * Phi wherever the switch scale_on_library_side puts the scale
+        (on the parameters it scales Sigma_w to S Sigma_w S, the same as scaling the basis columns)"""
+        b = self._scaled_basis_learnable()
+        return b if self.phase_gn.assume["scale_on_library_side"] else b * self.dtype(self.weights_scale)
+
     def get_traj_pos(self):
         b = self._scaled_basis_learnable()
         w = self._weights()
@@ -688,6 +694,20 @@ class ProDMP(MPBase):
             s = s * self.basis_gn.auto_basis_scale_factors
         return s
 
+    def _param_scale(self):
+        """[K+1] weights_scale per weight, goal_scale for the goal: the factors the switch scale_on_library_side=False
+        moves from the basis onto the parameters"""
+        K = self.basis_gn.num_basis
+        sc = np.full(K + 1, float(self.weights_scale))
+        sc[K] = float(self.goal_scale)
+        return sc
+
+    def cov_basis(self):
+        """[T, K+1] basis of traj_pos_cov: pos_H with the scales wherever the switch scale_on_library_side puts them
+        (on the parameters they scale Sigma_w to S Sigma_w S, the same as scaling the basis columns)"""
+        pos_H = self.tables()[0]
+        return pos_H if self.phase_gn.assume["scale_on_library_side"] else pos_H * self._param_scale()
+
     def _full_params(self):
         K = self.basis_gn.num_basis
         lead = self.params.shape[:-1]
@@ -700,8 +720,7 @@ class ProDMP(MPBase):
             p = np.concatenate([p, np.zeros((*lead, self.num_dof, 1))], axis=-1)
         A = self.phase_gn.assume
         if not A["scale_on_library_side"]:
-            sc = np.full(K + 1, float(self.weights_scale))
-            sc[K] = float(self.goal_scale)
+            sc = self._param_scale()
             p = (p.astype(F32) * sc.astype(F32)).astype(F32).astype(F64) if self.mode != "gold" else p * sc
         if self.goal_offset:
             p = p.copy()
@@ -818,7 +837,7 @@ def get_trajectory_generator(trajectory_generator_type, action_dim, basis_genera
 # trajectory covariance (App. B.5) — PARITY UNPINNED: mp_pytorch is absent and fancy_gym never calls it
 def traj_pos_cov(basis, params_L, num_dof, reg=1e-4, batch_scope=None):
     """Sigma_y = Psi (L L^T) Psi^T + reg * max(diag Sigma_y) * I in float64.
-    basis [T, Kc] (already scaled: weights_scale * Phi for ProMP, the bracketed H = [H_w | H_g] for ProDMP),
+    basis [T, Kc] (already scaled: weights_scale * Phi for ProMP, the bracketed H = [H_w | H_g] for ProDMP; `cov_basis()`),
     params_L [B, D, D] with D = num_dof * Kc (lower triangle used), rows / columns dof-major (d * T + t).
     Returns (cov [B, dof*T, dof*T], std [B, T, dof]); the max is per env unless batch_scope (mp_pytorch takes torch.max
     over whatever batch it is given; the reference never batches)."""

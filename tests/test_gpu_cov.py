@@ -33,9 +33,7 @@ def _oracle_basis(env_id, D):
     otg.set_params(np.zeros((1, D)))
     otg.set_initial_conditions(np.array(0.0), orc.env.current_pos, orc.env.current_vel)
     otg.set_duration(2.0, 0.01)
-    if env_id.startswith("fancy_ProMP"):
-        return np.asarray(otg._scaled_basis_learnable(), dtype=np.float64)
-    return np.asarray(otg.tables()[0], dtype=np.float64)
+    return np.asarray(otg.cov_basis(), dtype=np.float64)
 
 
 @pytest.mark.parametrize("env_id,B", [("fancy_ProMP/HoleReacher-v0", 3), ("fancy_ProDMP/SimpleReacher-v0", 17),
