@@ -11,6 +11,9 @@ import os
 FG_MAX_DOF = 8
 FG_MAX_OBS = 40
 FG_MAX_PLANS = 32
+# link counts the reacher rollout (fg_dispatch.cu) and env-step (fg_env_step.cu) kernels are instantiated for; resets and
+# stand-alone trajectories take 1..FG_MAX_DOF
+STEP_LINKS = range(2, 8)
 
 # enums (include/fancy_gym_b200.h)
 ENV_HOLE_REACHER, ENV_VIAPOINT_REACHER, ENV_SIMPLE_REACHER, ENV_TOY = 0, 1, 2, 3
@@ -155,6 +158,14 @@ def _load():
 
 lib = _load()
 assert lib.fg_abi_version() == 2, "ABI version mismatch between fancy_gym_b200/_lib.py and the shared library"
+
+
+def check_step_links(env_kind: int, n_links: int):
+    """Refuses a step of a reacher whose link count has no step kernel, before the caller changes any state (the library
+    refuses it too, but only once the host has counted the plan and flipped its result buffers)."""
+    if env_kind != ENV_TOY and n_links not in STEP_LINKS:
+        raise NotImplementedError(f"n_links={n_links}: the reacher step kernels are instantiated for "
+                                  f"{STEP_LINKS[0]}..{STEP_LINKS[-1]} links")
 
 
 def check(status: int):

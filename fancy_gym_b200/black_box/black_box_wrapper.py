@@ -471,6 +471,7 @@ class BlackBoxWrapper(Wrapper):
 
     def step(self, action, _keep_state: bool = False, _state=None):
         base = self._base
+        _lib.check_step_links(base.env_kind, base.n_links)
         params, as_numpy, scalar = self._prepare_params(action)
         self._set_plan(params)
         local = self.traj_gen.params.contiguous()
@@ -669,6 +670,7 @@ class BlackBoxWrapper(Wrapper):
         followed inside the kernel); use it when the plans do not depend on the observations in between (open-loop
         sequences, population-based search over plan sequences).  Falls back to a loop over step() where the plans cannot be
         laid out in advance (state-dependent schedule, learned tau / delay, verbose >= 2, trajectory hooks)."""
+        _lib.check_step_links(self._base.env_kind, self._base.n_links)
         a = actions if torch.is_tensor(actions) else torch.as_tensor(np.asarray(actions))
         if a.dim() == 2 and self.num_envs == 1:
             a = a[None]

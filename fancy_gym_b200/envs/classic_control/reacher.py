@@ -236,6 +236,7 @@ class BaseReacherEnv(Env):
         import ctypes as C
         if not self._was_reset:
             raise RuntimeError("Cannot call env.step() before calling env.reset()")
+        _lib.check_step_links(self.env_kind, self.n_links)
         a = action if torch.is_tensor(action) else torch.as_tensor(np.ascontiguousarray(action))
         if a.dtype not in (torch.float32, torch.float64):
             raise TypeError(f"action dtype must be float32 or float64, got {a.dtype}")

@@ -162,26 +162,65 @@ RANDOM_CASES += [("fancy_ProMP/HoleReacher-v0", 0.5, dict(rew_fct="vel_acc")), (
                  ("fancy_ProMP/HoleReacher-v0", 1.0, dict(allow_self_collision=True)),
                  ("fancy_ProMP/HoleReacher-v0", 1.0, dict(allow_wall_collision=True, hole_x=1.0, hole_width=0.4, hole_depth=0.7)),
                  ("fancy_DMP/ViaPointReacher-v0", 1.0, dict(allow_self_collision=True, random_start=True))]
+# Every link count the rollout is compiled for (fg_rollout_{env}_{2..7}.cu), for every MP: the link count sets the slot
+# layout, the shared-memory budget (opt-in above 48 KB at 6-7 links, which changes the occupancy and the work-queue grid), the
+# self-collision screen and pair loops, the per-link wall test and the observation compaction.  sigma per env is chosen so
+# that the comparison sees what it covers: wall collisions at every N and self collisions at N >= 4 (HoleReacher), self
+# collisions at N >= 4 (ViaPointReacher); asserted in the test.
+LINK_SIGMA = {"HoleReacher-v0": 2.0, "ViaPointReacher-v0": 3.0, "SimpleReacher-v0": 1.0}
+REGISTERED_LINKS = {"HoleReacher-v0": 5, "ViaPointReacher-v0": 5, "SimpleReacher-v0": 2}
+_POS = {"controller_kwargs": {"controller_type": "position"}}       # the run-time-K variant with the last desired position
+RANDOM_CASES += [(f"fancy_{mp}/{name}", s, dict(n_links=n)) for name, s in LINK_SIGMA.items() for n in range(2, 8)
+                 for mp in ("ProMP", "DMP", "ProDMP") if n != REGISTERED_LINKS[name]]
+RANDOM_CASES += [(f"fancy_ProMP/{name}", s, dict(n_links=n), _POS) for name, s in LINK_SIGMA.items() for n in (3, 7)]
 
 
-@pytest.mark.parametrize("env_id,sigma,env_over", RANDOM_CASES,
-                         ids=[f"{c[0]}-{c[1]}" + "".join(f"-{k}={v}" for k, v in c[2].items()) for c in RANDOM_CASES])
-def test_rollout_matches_oracle_random(env_id, sigma, env_over):
+def _collision_kinds(orc, ended):
+    """(wall hits, link-pair self hits) in the oracle's final state of the envs in `ended` (the state each episode ended in)"""
+    from oracle.reacher import CCW_EPS, _cross, forward_kinematics, wall_collision
+    e = orc.env
+    q = e.q[ended]
+    J = forward_kinematics(q)
+    pair = np.zeros(len(q), bool)
+    for i in range(e.n_links):
+        for j in range(i + 2, e.n_links):
+            A, Bp, C, D = J[:, i], J[:, i + 1], J[:, j], J[:, j + 1]
+            pair |= (((_cross(A, C, D) > CCW_EPS) != (_cross(Bp, C, D) > CCW_EPS))
+                     & ((_cross(A, Bp, C) > CCW_EPS) != (_cross(A, Bp, D) > CCW_EPS)))
+    wall = 0
+    if e.kind == "hole":
+        wall = int(wall_collision(q, e.hole_x[ended], e.hole_w[ended], e.hole_d[ended], margins=False)[0].sum())
+    return wall, int(pair.sum())
+
+
+@pytest.mark.parametrize("env_id,sigma,env_over,mp_over", [c + ({},) * (4 - len(c)) for c in RANDOM_CASES],
+                         ids=[f"{c[0]}-{c[1]}" + "".join(f"-{k}={v}" for k, v in c[2].items()) + ("-position" if len(c) > 3 else "")
+                              for c in RANDOM_CASES])
+def test_rollout_matches_oracle_random(env_id, sigma, env_over, mp_over):
     fancy_gym = _fg()
     B = 2048 + 37 if not env_over and env_id in P_OF else 512 + 5
-    env = fancy_gym.make(env_id, num_envs=B, device="cuda:0", **env_over)
+    env = fancy_gym.make(env_id, num_envs=B, device="cuda:0", mp_config_override=mp_over, **env_over)
     env.reset(seed=100)
     rng = np.random.default_rng(11)
-    params = (sigma * rng.standard_normal((B, n_params_of(env_id)))).astype(np.float32)
+    params = (sigma * rng.standard_normal((B, n_params_of(env_id, {"env": env_over})))).astype(np.float32)
     obs, ret, te, tr, info = env.step(torch.as_tensor(params, device="cuda:0"))
     obs, ret, te, tr = obs.cpu().numpy(), ret.cpu().numpy(), te.cpu().numpy(), tr.cpu().numpy()
     length = info["trajectory_length"].cpu().numpy()
 
-    orc = make_oracle(env_id, mode="mirror", mp_overrides={"env": env_over})
+    orc = make_oracle(env_id, mode="mirror", mp_overrides={"env": env_over, "ctrl": mp_over.get("controller_kwargs", {})})
     orc.reset(seeds=100 + np.arange(B))
     o_obs, o_ret, o_te, o_tr, o_info = orc.step(params)
     tie = o_info["min_margin"] < TIE_EPS
     agree = (length == o_info["trajectory_length"]) & (te == o_te) & (tr == o_tr)
+    n = env.unwrapped.n_links
+    if "n_links" in env_over:
+        wall, pair = _collision_kinds(orc, o_te)
+        print(f"{env_id} n_links={n}: {wall} wall / {pair} self collisions, {int(tie.sum())} boundary ties, "
+              f"{int((~agree).sum())} resolved differently")
+        if "HoleReacher" in env_id:
+            assert wall > 0 and (pair > 0 or n < 4), (wall, pair)
+        if "ViaPointReacher" in env_id:
+            assert pair > 0 or n < 4, pair
     assert (agree | tie).all(), f"{(~(agree | tie)).sum()} flag/length mismatches outside boundary ties"
     assert (~agree).sum() <= max(2, B // 500), f"too many boundary ties resolved differently: {(~agree).sum()}"
     m = agree
@@ -213,20 +252,22 @@ def _run(env, params, seed):
 
 def test_wall_modes_agree_at_full_size():
     """The transition-search wall test (mode 0: estimate + fix-up, mode 3: bisection) must give exactly the flags of the
-    literal 100-samples-per-link evaluation (mode 1: with the exact skip of links above ground, mode 2: no skipping at all)."""
+    literal 100-samples-per-link evaluation (mode 1: with the exact skip of links above ground, mode 2: no skipping at all),
+    at the registered 5 links and at link counts with other per-link loops and shared-memory budgets."""
     fancy_gym = _fg()
     B = 65536
-    gen = torch.Generator(device="cuda:0").manual_seed(0)
-    params = torch.randn(B, 25, generator=gen, device="cuda:0")
-    outs = []
-    for mode in (0, 1, 2, 3):
-        env = fancy_gym.make("fancy_ProMP/HoleReacher-v0", num_envs=B, device="cuda:0", context_sampler="device",
-                             mp_config_override={"black_box_kwargs": {"wall_mode": mode}})
-        outs.append(_run(env, params, 7))
-    for o in outs[1:]:
-        for a, b in zip(outs[0], o):
-            assert torch.equal(a, b)
-    assert int(outs[0][2].sum()) > B // 10      # the comparison saw many collisions
+    for n_links in (5, 2, 3, 7):
+        gen = torch.Generator(device="cuda:0").manual_seed(0)
+        params = torch.randn(B, 5 * n_links, generator=gen, device="cuda:0")
+        outs = []
+        for mode in (0, 1, 2, 3):
+            env = fancy_gym.make("fancy_ProMP/HoleReacher-v0", num_envs=B, device="cuda:0", context_sampler="device",
+                                 mp_config_override={"black_box_kwargs": {"wall_mode": mode}}, n_links=n_links)
+            outs.append(_run(env, params, 7))
+        for o in outs[1:]:
+            for a, b in zip(outs[0], o):
+                assert torch.equal(a, b), n_links
+        assert int(outs[0][2].sum()) > B // 10, n_links     # the comparison saw many collisions
 
 
 def test_determinism_and_shard_equivalence():
@@ -255,17 +296,19 @@ def test_determinism_and_shard_equivalence():
 
 def test_zero_params_keep_the_arm_still():
     """All-zero ProMP weights: zero velocity, the straight arm never collides with itself (collinear links,
-    exact zeros in the orientation tests), 200 steps, return == -dist^2 of the start pose."""
+    exact zeros in the orientation tests), 200 steps, return == -dist^2 of the start pose — at every link count the
+    rollout is compiled for (a check that does not rest on the oracle, which is pinned at the registered counts only)."""
     fancy_gym = _fg()
     B = 1024
-    env = fancy_gym.make("fancy_ProMP/HoleReacher-v0", num_envs=B, device="cuda:0")
-    env.reset(seed=0)
-    ee0 = env.unwrapped.end_effector()
-    goal = torch.stack([env.unwrapped.ctx[:, 0], -env.unwrapped.ctx[:, 2]], dim=1)
-    obs, ret, te, tr, info = env.step(torch.zeros(B, 25, device="cuda:0"))
-    assert bool((info["trajectory_length"] == 200).all()) and not bool(te.any()) and bool(tr.all())
-    want = -((ee0 - goal) ** 2).sum(1)
-    assert torch.allclose(ret, want, rtol=1e-12, atol=0)
+    for n_links in range(2, 8):
+        env = fancy_gym.make("fancy_ProMP/HoleReacher-v0", num_envs=B, device="cuda:0", n_links=n_links)
+        env.reset(seed=0)
+        ee0 = env.unwrapped.end_effector()
+        goal = torch.stack([env.unwrapped.ctx[:, 0], -env.unwrapped.ctx[:, 2]], dim=1)
+        obs, ret, te, tr, info = env.step(torch.zeros(B, 5 * n_links, device="cuda:0"))
+        assert bool((info["trajectory_length"] == 200).all()) and not bool(te.any()) and bool(tr.all()), n_links
+        want = -((ee0 - goal) ** 2).sum(1)
+        assert torch.allclose(ret, want, rtol=1e-12, atol=0), n_links
 
 
 # --------------------------------------------------------------------------------------------
@@ -276,6 +319,10 @@ RESET_CASES = [("fancy/HoleReacher-v0", {}), ("fancy/HoleReacher-v0", dict(hole_
                ("fancy/ViaPointReacher-v0", {}), ("fancy/ViaPointReacher-v0", dict(random_start=True, target=(3.0, 2.0))),
                ("fancy/SimpleReacher-v0", {}), ("fancy/SimpleReacher-v0", dict(random_start=False)),
                ("fancy/LongSimpleReacher-v0", dict(target=(1.0, -2.0)))]
+# every link count fg_reset takes: the observation layout and, for ViaPointReacher / SimpleReacher, the radii of the
+# rejection samplers (total = n_links) follow it
+RESET_CASES += [(f"fancy/{name}", dict(n_links=n)) for name in REGISTERED_LINKS for n in range(1, 9)      # 1..FG_MAX_DOF
+                if n != REGISTERED_LINKS[name]]
 
 
 @pytest.mark.parametrize("env_id,kw", RESET_CASES, ids=[f"{c[0]}-{i}" for i, c in enumerate(RESET_CASES)])
@@ -315,25 +362,33 @@ def test_blackbox_reset_fast_path_matches_wrapper_chain():
 # --------------------------------------------------------------------------------------------
 # per-env learned tau / delay (SURVEY §8f rank 2): basis evaluated in the kernel, rollout from the HBM trajectory
 # --------------------------------------------------------------------------------------------
-@pytest.mark.parametrize("env_id,phase", [("fancy_ProMP/HoleReacher-v0", dict(learn_tau=True, learn_delay=True)),
-                                          ("fancy_ProMP/HoleReacher-v0", dict(learn_delay=True)),
-                                          ("fancy_DMP/ViaPointReacher-v0", dict(learn_tau=True)),
-                                          ("fancy_DMP/HoleReacher-v0", dict(learn_tau=True, learn_delay=True)),
-                                          ("fancy_ProMP/SimpleReacher-v0", dict(learn_tau=True)),
-                                          ("fancy_ProDMP/SimpleReacher-v0", dict(learn_tau=True)),
-                                          ("fancy_ProDMP/HoleReacher-v0", dict(learn_tau=True, learn_delay=True))],
-                         ids=["promp-tau-delay", "promp-delay", "dmp-tau", "dmp-tau-delay", "promp-pd-tau", "prodmp-tau",
-                              "prodmp-tau-delay"])
-def test_per_env_tau_delay_matches_oracle(env_id, phase):
+_TAU_DELAY = dict(learn_tau=True, learn_delay=True)
+PHASE_CASES = [("promp-tau-delay", "fancy_ProMP/HoleReacher-v0", _TAU_DELAY, {}),
+               ("promp-delay", "fancy_ProMP/HoleReacher-v0", dict(learn_delay=True), {}),
+               ("dmp-tau", "fancy_DMP/ViaPointReacher-v0", dict(learn_tau=True), {}),
+               ("dmp-tau-delay", "fancy_DMP/HoleReacher-v0", _TAU_DELAY, {}),
+               ("promp-pd-tau", "fancy_ProMP/SimpleReacher-v0", dict(learn_tau=True), {}),
+               ("prodmp-tau", "fancy_ProDMP/SimpleReacher-v0", dict(learn_tau=True), {}),
+               ("prodmp-tau-delay", "fancy_ProDMP/HoleReacher-v0", _TAU_DELAY, {})]
+# fg_trajgen_phase + the trajectory-from-HBM rollout at link counts the in-rollout phase is not instantiated for
+PHASE_CASES += [(f"{mp.lower()}-tau-delay-{name}-{n}links", f"fancy_{mp}/{name}", _TAU_DELAY, dict(n_links=n))
+                for mp, name in (("ProMP", "HoleReacher-v0"), ("DMP", "ViaPointReacher-v0"), ("ProDMP", "SimpleReacher-v0"))
+                for n in (3, 7)]
+
+
+@pytest.mark.parametrize("env_id,phase,env_over", [c[1:] for c in PHASE_CASES], ids=[c[0] for c in PHASE_CASES])
+def test_per_env_tau_delay_matches_oracle(env_id, phase, env_over):
     fancy_gym = _fg()
     B = 300 + 7
     mp_type = "promp" if "ProMP" in env_id else ("prodmp" if "ProDMP" in env_id else "dmp")
     base_phase = dict(RESOLVED_PHASE(env_id), **phase)
-    env = fancy_gym.make(env_id, num_envs=B, device="cuda:0", mp_config_override={"phase_generator_kwargs": base_phase})
+    env = fancy_gym.make(env_id, num_envs=B, device="cuda:0", mp_config_override={"phase_generator_kwargs": base_phase},
+                         **env_over)
+    assert not env._phase_fusable() or not env_over         # (other link counts: phase kernel, then the rollout from HBM)
     env.reset(seed=50)
     rng = np.random.default_rng(4)
     n_extra = int(phase.get("learn_tau", False)) + int(phase.get("learn_delay", False))
-    params = (0.4 * rng.standard_normal((B, n_params_of(env_id) + n_extra))).astype(np.float32)
+    params = (0.4 * rng.standard_normal((B, n_params_of(env_id, {"env": env_over}) + n_extra))).astype(np.float32)
     i = 0
     if phase.get("learn_tau"):
         # partly outside tau_bound = [0.02, 2.0]: clipped like the reference (ProDMP pre-computes 6 tau: keep t / tau <= 6)
@@ -343,7 +398,7 @@ def test_per_env_tau_delay_matches_oracle(env_id, phase):
         params[:, i] = rng.uniform(0.0, 0.6, B)
     assert env.action_space.shape[0] == params.shape[1]
 
-    orc = make_oracle(env_id, mode="mirror", mp_overrides={"phase": phase})
+    orc = make_oracle(env_id, mode="mirror", mp_overrides={"phase": phase, "env": env_over})
     orc.reset(seeds=50 + np.arange(B))
     o_pos, o_vel = orc.get_trajectory(params)
     pos, vel = env.get_trajectory(torch.as_tensor(params, device="cuda:0"))

@@ -25,6 +25,10 @@ PLAN_CASES = [
     ("fancy_DMP/ViaPointReacher-v0", dict(replanning_schedule=lambda p, v, o, a, t: t % 30 == 0, max_planning_times=3), {}, 3, 1.0),
     ("fancy_ProMP/SimpleReacher-v0", dict(replanning_schedule=lambda p, v, o, a, t: t % 64 == 0, reward_aggregation=np.mean), {}, 4, 0.5),
 ]
+# plans inside one launch at link counts other than the registered ones: every env, re-planning with condition_on_desired
+PLAN_CASES += [(env_id, dict(replanning_schedule=lambda p, v, o, a, t: t % 40 == 0, condition_on_desired=True), dict(n_links=n), 5, 0.5)
+               for env_id in ("fancy_DMP/HoleReacher-v0", "fancy_DMP/ViaPointReacher-v0", "fancy_ProDMP/SimpleReacher-v0")
+               for n in (3, 7)]
 
 
 def _eq(a, b):
@@ -268,20 +272,25 @@ def test_vector_env_applies_the_learned_tau_of_every_new_episode():
 
 
 # ---- per-env learned tau / delay evaluated inside the rollout (fg_rollout_io.phase) ---------------------------------------
+_LIN_TAU_DELAY = {"phase_generator_kwargs": dict(phase_generator_type="linear", learn_tau=True, learn_delay=True)}
+_EXP_TAU = {"phase_generator_kwargs": dict(phase_generator_type="exp", alpha_phase=2, learn_tau=True)}
 FUSED_PHASE_CASES = [
-    ("fancy_ProMP/HoleReacher-v0", {"phase_generator_kwargs": dict(phase_generator_type="linear", learn_tau=True, learn_delay=True)}, {}),
-    ("fancy_ProMP/HoleReacher-v0", {"phase_generator_kwargs": dict(phase_generator_type="linear", learn_delay=True)}, {}),
-    ("fancy_DMP/ViaPointReacher-v0", {"phase_generator_kwargs": dict(phase_generator_type="exp", alpha_phase=2, learn_tau=True)}, {}),
-    ("fancy_DMP/HoleReacher-v0", {"phase_generator_kwargs": dict(phase_generator_type="exp", alpha_phase=2.5, learn_tau=True, learn_delay=True)}, {}),
-    ("fancy_ProMP/SimpleReacher-v0", {"phase_generator_kwargs": dict(phase_generator_type="linear", learn_tau=True)}, {}),
-    ("fancy_DMP/LongSimpleReacher-v0", {"phase_generator_kwargs": dict(phase_generator_type="exp", alpha_phase=2, learn_tau=True)}, {}),
-    ("fancy_ProMP/HoleReacher-v0", {}, {"learn_sub_trajectories": True}),
-    ("fancy_DMP/ViaPointReacher-v0", {}, {"learn_sub_trajectories": True, "condition_on_desired": True}),
+    ("fancy_ProMP/HoleReacher-v0", _LIN_TAU_DELAY, {}, {}),
+    ("fancy_ProMP/HoleReacher-v0", {"phase_generator_kwargs": dict(phase_generator_type="linear", learn_delay=True)}, {}, {}),
+    ("fancy_DMP/ViaPointReacher-v0", _EXP_TAU, {}, {}),
+    ("fancy_DMP/HoleReacher-v0", {"phase_generator_kwargs": dict(phase_generator_type="exp", alpha_phase=2.5, learn_tau=True, learn_delay=True)}, {}, {}),
+    ("fancy_ProMP/SimpleReacher-v0", {"phase_generator_kwargs": dict(phase_generator_type="linear", learn_tau=True)}, {}, {}),
+    ("fancy_DMP/LongSimpleReacher-v0", _EXP_TAU, {}, {}),
+    ("fancy_ProMP/HoleReacher-v0", {}, {"learn_sub_trajectories": True}, {}),
+    ("fancy_DMP/ViaPointReacher-v0", {}, {"learn_sub_trajectories": True, "condition_on_desired": True}, {}),
+    # the in-rollout phase is instantiated for 5 and 2 links: the velocity-controlled envs at 2
+    ("fancy_ProMP/HoleReacher-v0", _LIN_TAU_DELAY, {}, dict(n_links=2)),
+    ("fancy_DMP/ViaPointReacher-v0", _EXP_TAU, {}, dict(n_links=2)),
 ]
 
 
-@pytest.mark.parametrize("env_id,over,bbk", FUSED_PHASE_CASES, ids=[f"{c[0]}-{i}" for i, c in enumerate(FUSED_PHASE_CASES)])
-def test_phase_inside_the_rollout_equals_trajgen_then_rollout(env_id, over, bbk, monkeypatch):
+@pytest.mark.parametrize("env_id,over,bbk,env_kw", FUSED_PHASE_CASES, ids=[f"{c[0]}-{i}" for i, c in enumerate(FUSED_PHASE_CASES)])
+def test_phase_inside_the_rollout_equals_trajgen_then_rollout(env_id, over, bbk, env_kw, monkeypatch):
     """the basis of a per-env phase evaluated by the rollout thread itself == fg_trajgen_phase writing the trajectory to HBM and
     a FG_MP_TRAJ rollout reading it back: bit for bit, incl. ragged sub-trajectory plans and condition_on_desired"""
     import fancy_gym_b200 as fancy_gym
@@ -289,8 +298,8 @@ def test_phase_inside_the_rollout_equals_trajgen_then_rollout(env_id, over, bbk,
     cfg = dict(over)
     if bbk:
         cfg["black_box_kwargs"] = dict(bbk)
-    fused = fancy_gym.make(env_id, num_envs=B, device=DEV, mp_config_override=cfg)
-    split = fancy_gym.make(env_id, num_envs=B, device=DEV, mp_config_override=cfg)
+    fused = fancy_gym.make(env_id, num_envs=B, device=DEV, mp_config_override=cfg, **env_kw)
+    split = fancy_gym.make(env_id, num_envs=B, device=DEV, mp_config_override=cfg, **env_kw)
     assert fused._phase_fusable()
     fused.reset(seed=9); split.reset(seed=9)
     gen = torch.Generator(device=DEV).manual_seed(4)

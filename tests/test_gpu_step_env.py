@@ -96,6 +96,10 @@ REPLAY_CASES += [("fancy_ProMP/HoleReacher-v0", dict(rew_fct="vel_acc"), {}),
                  ("fancy_DMP/ViaPointReacher-v0", dict(allow_self_collision=True), {}),
                  ("fancy_ProMP/HoleReacher-v0", {}, _POS), ("fancy_DMP/ViaPointReacher-v0", {}, _POS),
                  ("fancy_ProDMP/SimpleReacher-v0", {}, _POS)]
+# every k_env_step instantiation against the verbose=2 instantiation of k_rollout at the same link count, under every MP
+_REGISTERED_LINKS = {"HoleReacher-v0": 5, "ViaPointReacher-v0": 5, "SimpleReacher-v0": 2}
+REPLAY_CASES += [(f"fancy_{mp}/{name}", dict(n_links=n), {}) for name in _REGISTERED_LINKS for n in range(2, 8)
+                 for mp in ("ProMP", "DMP", "ProDMP") if n != _REGISTERED_LINKS[name]]
 
 
 @pytest.mark.parametrize("env_id,env_over,mp_over", REPLAY_CASES,
@@ -153,6 +157,10 @@ ORACLE_CASES = [("HoleReacher-v0", 2.0, {}, "float32"), ("HoleReacher-v0", 2.0, 
                 ("ViaPointReacher-v0", 2.0, dict(allow_self_collision=True, random_start=True), "float32"),
                 ("SimpleReacher-v0", 30.0, {}, "float32"), ("SimpleReacher-v0", 30.0, {}, "float64"),
                 ("LongSimpleReacher-v0", 30.0, dict(random_start=False), "float64")]
+# every link count k_env_step is instantiated for; the action dtype alternates with it, so both run for every env
+_SIGMA = {"HoleReacher-v0": 2.0, "ViaPointReacher-v0": 2.0, "SimpleReacher-v0": 30.0}
+ORACLE_CASES += [(name, _SIGMA[name], dict(n_links=n), ("float32", "float64")[n % 2])
+                 for name in _REGISTERED_LINKS for n in range(2, 8) if n != _REGISTERED_LINKS[name]]
 _KIND = {"HoleReacher-v0": "hole", "ViaPointReacher-v0": "viapoint", "SimpleReacher-v0": "simple", "LongSimpleReacher-v0": "simple"}
 
 
@@ -193,6 +201,16 @@ def test_step_env_matches_oracle_at_scale(name, sigma, over, dtype):
         o_ob, o_r, o_te, o_info = orc.step(a)
         ob, r, te, tr = ob.cpu().numpy(), r.cpu().numpy(), te.cpu().numpy(), tr.cpu().numpy()
         assert (np.abs(ob - o_ob) <= 1e-5 * np.maximum(1.0, np.abs(o_ob))).all(), t
+        # without the oracle (pinned against the reference at the registered link counts only): the observation's joint
+        # entries and the end effector follow from the env's own float64 state
+        n, q = env.n_links, env.q.cpu().numpy()
+        trig = np.concatenate([np.cos(q), np.sin(q)], axis=1).astype(np.float32)
+        assert (np.abs(ob[:, :2 * n] - trig) <= np.spacing(np.abs(trig))).all(), t          # within one float32 ulp
+        assert np.array_equal(ob[:, 2 * n:3 * n], env.v.cpu().numpy().astype(np.float32)), t
+        if "end_effector" in info:
+            th = np.cumsum(q, axis=1)
+            ee = np.stack([np.cos(th).sum(axis=1), np.sin(th).sum(axis=1)], axis=1)
+            assert rel_err(info["end_effector"].cpu().numpy(), ee).max() <= 1e-12, t
         assert (tr == (t + 1 >= 200)).all(), t
         agree = te == o_te
         for k_ in ("is_success", "is_collided"):

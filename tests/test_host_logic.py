@@ -389,3 +389,16 @@ def test_rbf_recurrence_error_stays_far_inside_the_tie_margin():
         phi /= phi.sum(1, keepdims=True)
         rel = np.abs(phi - direct) / direct
         assert rel.max() < 2.0 ** -40 / 8, rel.max()          # margin of the fall-back: 2**12 ulps = 2**-40 relative
+
+
+# ---- link counts the step kernels exist for ---------------------------------------------------------------------------
+def test_step_link_range_is_checked_on_the_host():
+    from fancy_gym_b200 import _lib
+    for kind in (_lib.ENV_HOLE_REACHER, _lib.ENV_VIAPOINT_REACHER, _lib.ENV_SIMPLE_REACHER):
+        for n in range(1, _lib.FG_MAX_DOF + 1):
+            if n in _lib.STEP_LINKS:
+                _lib.check_step_links(kind, n)
+            else:
+                with pytest.raises(NotImplementedError, match=r"n_links=%d: .* 2\.\.7 links" % n):
+                    _lib.check_step_links(kind, n)
+    _lib.check_step_links(_lib.ENV_TOY, 1)          # the test env has its own instantiations (1, 2, 5)
