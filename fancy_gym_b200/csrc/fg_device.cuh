@@ -272,21 +272,38 @@ __device__ __noinline__ bool self_hits_accurate(const Angles<N> a) {
   return self_hits<N, true>(a.th, zero, zero, unused);
 }
 
+// max / min that return NaN if either operand is NaN (PTX max.NaN / min.NaN, sm_80+; fmaxf / fminf return the other one):
+// one FMNMX each, like fmaxf / fminf, and the same result for every other operand
+__device__ __forceinline__ float fmax_nan(float a, float b) {
+  float r;
+  asm("max.NaN.f32 %0, %1, %2;" : "=f"(r) : "f"(a), "f"(b));
+  return r;
+}
+__device__ __forceinline__ float fmin_nan(float a, float b) {
+  float r;
+  asm("min.NaN.f32 %0, %1, %2;" : "=f"(r) : "f"(a), "f"(b));
+  return r;
+}
+
 // any(q > pi) or any(q < -pi) (base_reacher.py:111): |q| > pi as an unsigned compare of the sign-stripped bit patterns
 // (non-negative doubles order like integers).  Fast screen on the HIGH words only: non-negative float patterns order like the
-// integers they are, so the largest sign-stripped high word is one FMNMX(3) chain with |.| modifiers; only when it reaches pi's
-// high word (|q| within 2^-20 of pi or beyond: rare) are the full 64-bit patterns compared.
+// integers they are, so the largest sign-stripped high word is one FMNMX chain with |.| modifiers; only when it reaches pi's
+// high word (|q| within 2^-20 of pi or beyond: rare) are the full 64-bit patterns compared.  The high word of |q| >= 2^1017
+// (inf included) read as a float32 is a NaN: the max keeps it and the screen lets it through.  A NaN joint is not a limit
+// (NaN > pi is False): its pattern lies above inf's.
 template <int N>
 __device__ __forceinline__ bool joint_limits(const double (&q)[N]) {
   bool lim = false;
-  constexpr unsigned long long kPiBits = 0x400921FB54442D18ULL;
+  constexpr unsigned long long kPiBits = 0x400921FB54442D18ULL, kInfBits = 0x7FF0000000000000ULL;
   float hi_max = 0.f;
 #pragma unroll
-  for (int i = 0; i < N; ++i) hi_max = fmaxf(hi_max, fabsf(__int_as_float(__double2hiint(q[i]))));
-  if (hi_max >= __int_as_float(0x400921FB)) {
+  for (int i = 0; i < N; ++i) hi_max = fmax_nan(hi_max, fabsf(__int_as_float(__double2hiint(q[i]))));
+  if (!(hi_max < __int_as_float(0x400921FB))) {
 #pragma unroll
-    for (int i = 0; i < N; ++i)
-      lim |= ((unsigned long long)__double_as_longlong(q[i]) & 0x7FFFFFFFFFFFFFFFULL) > kPiBits;
+    for (int i = 0; i < N; ++i) {
+      const unsigned long long bits = (unsigned long long)__double_as_longlong(q[i]) & 0x7FFFFFFFFFFFFFFFULL;
+      lim |= (bits > kPiBits) & (bits <= kInfBits);
+    }
   }
   return lim;
 }

@@ -754,7 +754,8 @@ k_rollout(const __grid_constant__ DevCfg c, const __grid_constant__ fg_rollout_i
 #pragma unroll
           for (int i = 0; i < N; ++i) {
             const float des = (VEL_ONLY || c.ctrl == FG_CTRL_VELOCITY) ? vel[i] : pos[i];
-            a32[i] = fminf(fmaxf(des, -c.act_lim), c.act_lim);
+            // np.clip(des, -lim, lim) keeps a NaN, which fminf / fmaxf would turn into -lim
+            a32[i] = fmin_nan(fmax_nan(des, -c.act_lim), c.act_lim);
             a64[i] = (double)a32[i];
           }
         }
